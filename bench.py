@@ -2,6 +2,7 @@
 """bench.py — alert cells / second to a converged, quorum-decided cut (BASELINE.json's metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c5|c4|c3|c2] [--nodes n]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic alert stream, from an empty detector to the decision:
     [per batch] filter -> per-receiver cut detection (subject-bucketed kernels) -> implicit invalidation -> per-node proposal
@@ -28,6 +29,7 @@ Receivers are sharded over the GPUs by ring-0 range; the cluster size stays fixe
            the measured rate of that sample, the whole-cluster extrapolation is a labelled side field.
 """
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -69,7 +71,14 @@ def parse():
                         "checked on the device, batch-by-batch replay if refused) or as 8 separate calls")
     p.add_argument("--emulate-shard", type=int, default=0,
                    help="tuning aid: run rank 0's shard of a G-way run on ONE GPU without NCCL (no decision is reached)")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last timed step computed as DIR/<name>.npy (float32 / float64), to compare two builds "
+                        "output for output")
     a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     if a.nodes <= 0:
         a.nodes = DEFAULT_NODES[a.workload]
     return a
@@ -138,10 +147,16 @@ class Clocks:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.dev), "--query-gpu=" + self.Q,
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self._reap)        # a run that fails while the poller is stopped must not leave it behind
             threading.Thread(target=self._pump, daemon=True).start()
             self.first.wait(10.0)
         except OSError:
             self.proc = None
+
+    def _reap(self):
+        if self.proc.poll() is None:
+            self.proc.kill()
+        self.proc.wait()
 
     def _pump(self):
         for line in self.proc.stdout:
@@ -304,18 +319,14 @@ def run_reference(args):
     if rank != 0:
         return
     from oracle import oracle_py as orc
-    orc.build()
     threads = max(1, orc.hardware_threads())
     prob = CpuProblem(args)
     log("[reference] setup %.1fs (n=%d), %d threads" % (prob.setup_s, args.nodes, threads))
     vals = []
-    t_start = time.time()
     for i in range(args.warmup + args.steps):
         d, cells, upto = prob.measure(threads)
         if i >= args.warmup:
             vals.append(d)
-        if time.time() - t_start > 240 and vals:         # the whole run stays within a few minutes
-            break
     v = float(np.mean([x["value"] for x in vals]))
     d = dict(vals[-1])
     d["value"] = v
@@ -515,6 +526,8 @@ def run_ours(args):
     if os.environ.get("RAPID_B200_STEP_TIMES"):
         log("[rank %d] per-step host wall ms: %s" % (rank, " ".join("%.3f" % x for x in per_step)))
     check(res)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cl, res, begin, "rank%d_" % rank if G > 1 else "", G)
     prof_steps = max(2, min(args.steps, 5))
     for _ in range(prof_steps):
         check(step_profile())
@@ -651,13 +664,50 @@ def run_ours(args):
         if not args.no_cpu_baseline and G == 1:
             try:
                 from oracle import oracle_py as orc
-                orc.build()
                 line["cpu_baseline"] = CpuProblem(args).measure(max(1, orc.hardware_threads()))[0]
             except Exception as e:       # the baseline is a reported extra; never lose the GPU line over it
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "failed: %r" % (e,)}
         emit(line)
     if G > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_RECEIVERS = 1 << 20
+
+
+def dump_outputs(d, cl, res, begin, prefix, G):
+    """What the last timed step handed its caller, as DIR/<prefix><name>.npy:
+        decision.npy              FastPaxos.result(): decided, hash (hi, lo), hash2 (hi, lo), length, count, votes_received,
+                                  decided_in (-1: none)
+        cut.npy                   the decided proposal (node ids, as getProposal lists them) of the first receiver holding it
+        receivers.npy             ring-0 positions of the receivers the next three arrays describe
+        proposal_fingerprint.npy  VirtualCluster.readOutputs(): per receiver hash (hi, lo), hash2 (hi, lo)
+        proposal_len.npy, announced.npy
+    uint64 fingerprints are split into 32-bit halves so that float64 holds them exactly.  Above DUMP_MAX_RECEIVERS receivers
+    (over all ranks) a fixed seeded sample of them is written, which keeps the files under 64 MB."""
+    os.makedirs(d, exist_ok=True)
+    out = cl.readOutputs()
+    R, cap = len(out.proposal_len), DUMP_MAX_RECEIVERS // G
+    idx = np.arange(R) if R <= cap else np.sort(np.random.default_rng(0).choice(R, cap, replace=False))
+
+    def halves(h):
+        h = np.asarray(h, np.uint64)
+        return np.stack([h >> np.uint64(32), h & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+
+    holders = np.nonzero((out.proposal_hash == res.hash) & (out.proposal_hash2 == res.hash2) & (out.proposal_len == res.length))[0]
+    cut = cl.getProposal(int(holders[0])) if res.decided and len(holders) else []
+    arrays = {
+        "decision": np.concatenate([[float(res.decided)], halves([res.hash, res.hash2]).ravel(),
+                                    [res.length, res.count, res.votes_received, -1 if res.decided_in is None else res.decided_in]]),
+        "cut": np.asarray(cut, np.float64),
+        "receivers": (begin + idx).astype(np.float64),
+        "proposal_fingerprint": np.concatenate([halves(out.proposal_hash[idx]), halves(out.proposal_hash2[idx])], axis=1),
+        "proposal_len": out.proposal_len[idx].astype(np.float32),
+        "announced": out.announced[idx].astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(d, prefix + name + ".npy"), a)
+    log("outputs of the last timed step: %s (%d of %d receivers)" % (", ".join(prefix + k + ".npy" for k in arrays), len(idx), R))
 
 
 _JSON_OUT = None

@@ -119,10 +119,40 @@ def failure_detector_stream():
         json.dump(out, f)
 
 
+def xxh64_vectors():
+    """XXH64 digests from two implementations independent of the oracle: python-xxhash (bytes, and hashInt / hashLong as
+    little-endian bytes) and the system libxxhash.  Not oracle pins: tests/test_oracle_xxh64.py holds the oracle to them."""
+    import ctypes
+    import random
+    import struct
+    import xxhash
+    lx = ctypes.CDLL("libxxhash.so.0")
+    lx.XXH64.restype = ctypes.c_uint64
+    lx.XXH64.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint64]
+    rng = random.Random(7)
+    out = {"python_xxhash": {"version": xxhash.VERSION, "bytes": [], "int": [], "long": []}, "libxxhash": []}
+    for n in list(range(0, 80)) + [127, 128, 129, 1000]:
+        data = bytes(rng.getrandbits(8) for _ in range(n))
+        out["python_xxhash"]["bytes"].append([data.hex(), [[seed, xxhash.xxh64(data, seed=seed).intdigest()]
+                                                           for seed in (0, 1, 2, 9, 0xDEADBEEF, 2**63 + 5)]])
+    for seed in range(10):
+        for v in (0, 1, -1, 1234, 65535, 2**31 - 1, -(2**31)):
+            out["python_xxhash"]["int"].append([v, seed, xxhash.xxh64(struct.pack("<i", v), seed=seed).intdigest()])
+        for v in (0, 1, -1, 2**63 - 1, -(2**63), 0x0123456789ABCDEF):
+            out["python_xxhash"]["long"].append([v, seed, xxhash.xxh64(struct.pack("<q", v), seed=seed).intdigest()])
+    rng = random.Random(11)
+    for n in (0, 1, 3, 4, 7, 8, 9, 15, 31, 32, 33, 63, 64, 100):
+        data = bytes(rng.getrandbits(8) for _ in range(n))
+        out["libxxhash"].append([data.hex(), [[seed, lx.XXH64(data, n, seed)] for seed in (0, 3, 9)]])
+    with open(os.path.join(HERE, "xxh64_vectors.json"), "w") as f:
+        json.dump(out, f)
+
+
 if __name__ == "__main__":
     orc.build()
     ring_keys()
     cut_scenarios()
     paxos_rule_cases()
     failure_detector_stream()
+    xxh64_vectors()
     print("wrote", os.listdir(HERE))
